@@ -12,6 +12,9 @@ sample of a timed batch is answered by the oracle (CPU restatement of the refere
 `cpu_baseline` -- and the GPU's records for those queries must be identical (DocumentId order, Score bits, Tiebreaker bytes);
 a mismatch fails the run instead of printing a line.
 N > 1: see `run_ours` (one process per GPU under torchrun).
+--dump-outputs DIR: the records the `value` path returned for the last timed batch go to DIR/<name>.npy (see dump_outputs); the
+corpus and the query batches are seeded, so two builds run with the same arguments can be compared output for output. That path
+returns no facet tables (device-resident batches are uploaded without facet capacity), so none are written.
 """
 import argparse
 import json
@@ -89,6 +92,25 @@ def measured_peak():
     if os.path.exists(p):
         return float(json.load(open(p))["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
+
+
+DUMP_PAD = {"doc_key": -1, "score": 0, "tie": 0}
+
+
+def dump_outputs(out_dir, arrays):
+    """One DIR/<name>.npy per result array (names of ifx_batch_result): float32 as it is, integers as float64 (exact below 2**53).
+    Record slots at or beyond a query's n are never written by the library (their memory is undefined): they are saved as DUMP_PAD."""
+    n = arrays["n"]
+    arrays = dict(arrays)
+    for k, fill in DUMP_PAD.items():
+        v = arrays[k]; arrays[k] = np.where(np.arange(v.shape[1])[None, :] >= n[:, None], v.dtype.type(fill), v)
+    arrays = {k: v if v.dtype == np.float32 else v.astype(np.float64) for k, v in arrays.items()}
+    size = sum(v.nbytes for v in arrays.values())
+    if size > 64 << 20:                    # 10k queries x top-10: 2.2 MB
+        raise ValueError("%d bytes of outputs exceed the 64 MiB dump budget" % size)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def make_corpus(wl):
@@ -222,6 +244,7 @@ def run_sharded(args, wl, rank, world, local):
                 agg[k] += getattr(st, k)
             if first is None:
                 first = merged
+            last = merged
     exch = dict(eng.exchange_ms); host = dict(eng.host_ms)
     for u in ups:
         eng.FreeBatch(u)
@@ -239,6 +262,9 @@ def run_sharded(args, wl, rank, world, local):
     mx = tt.clone(); dist.all_reduce(mx, op=dist.ReduceOp.MAX); sm = tt.clone(); dist.all_reduce(sm)
     if rank != 0:
         dist.barrier(); dist.destroy_process_group(); return 0
+    if args.dump_outputs:                  # the merged records every rank holds
+        o_key, o_score, o_tie, o_n, total, status, _ = last
+        dump_outputs(args.dump_outputs, dict(doc_key=o_key, score=o_score, tie=o_tie, n=o_n, total_candidates=total, status=status))
     dev_t, e2e_t = float(mx[0]), float(mx[1]); algo_all = float(sm[2]); aggm = {k: float(mx[3 + i]) for i, k in enumerate(agg)}
     value = wl["nq"] * args.steps / dev_t; e2e = wl["nq"] * args.steps / e2e_t
     peak, peak_src = measured_peak(); s1_ms = aggm["ms_stage1"] / args.steps
@@ -321,6 +347,8 @@ def run_ours(args, wl, rank, world, local):
             algo += st.algo_bytes_stage1; launches += st.kernel_launches; q_max = max(q_max, st.s1_query_ms_max); q_sum += st.s1_query_ms_sum
             s1_info = {"queries_scored_per_warp": st.s1_light + st.s1_mid, "queries_scored_per_cta": st.s1_heavy, "waves": st.s1_waves, "staging_pool_bytes": int(st.s1_pool_bytes)}
     barrier()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, eng.DownloadBatch(handles[-1], wl["nq"], 10))
     for h in handles:
         eng.FreeBatch(h)
     # ---- e2e: host buffers in / out through the C-ABI call ifx_search_batch (query upload + result download inside the region) --
@@ -399,7 +427,12 @@ def main():
     ap.add_argument("--workload", default="c3", choices=list(WORKLOADS), help="default: c3 = BASELINE.json configs[2], the configuration the metric is quoted on")
     ap.add_argument("--ref-sample", type=int, default=512, help="queries per step of the CPU arms (bounded sample of the batch)")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the oracle leg (cpu_baseline + parity assertion)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the records of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the records of the CUDA path; it does not apply to --impl reference")
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":

@@ -362,6 +362,18 @@ class SearchEngine:
         self._check(self._gpu.ifx_batch_run(handle, C.byref(st)), "ifx_batch_run")
         return st
 
+    def DownloadBatch(self, handle, nq, cap):
+        """Records of the last RunBatch on `handle` (ifx_batch_download): doc_key / score / tie [nq, cap], n / total_candidates / status [nq].
+        `cap` >= the batch's largest MaxNumberOfRecordsToReturn. Row q holds n[q] records; the slots after them are undefined. An uploaded
+        batch has no facet capacity, so there are no facet tables to read back."""
+        out = _BatchResult(); out.cap = cap; out.facet_cap = 0
+        bufs = dict(doc_key=np.zeros((nq, cap), np.int64), score=np.zeros((nq, cap), np.float32), tie=np.zeros((nq, cap), np.uint8),
+                    n=np.zeros(nq, np.int32), total_candidates=np.zeros(nq, np.int32), status=np.zeros(nq, np.int32))
+        out.doc_key, out.score, out.tie = _p(bufs["doc_key"]), _p(bufs["score"]), _p(bufs["tie"])
+        out.n, out.total_candidates, out.status = _p(bufs["n"]), _p(bufs["total_candidates"]), _p(bufs["status"])
+        self._check(self._gpu.ifx_batch_download(handle, C.byref(out)), "ifx_batch_download")
+        return bufs
+
     def FreeBatch(self, handle):
         self._gpu.ifx_batch_free(handle)
 

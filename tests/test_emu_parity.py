@@ -41,6 +41,11 @@ def test_emu_synthetic(emu, multi):
     eng, orc = build_pair(docs["keys"], schema, cols, gpu_lib=emu)
     assert not compare_stage1(eng, orc, qs)
     assert not compare_search(eng, orc, qs)
+    # the split form (upload, run, read back) returns the records ifx_search_batch just returned for the same batch
+    h = eng.UploadBatch([ib.Query(q, 10) for q in qs]); eng.RunBatch(h); got = eng.DownloadBatch(h, len(qs), 10); eng.FreeBatch(h)
+    want = dict(zip(("doc_key", "score", "tie", "n", "total_candidates", "status"), eng.last_raw))
+    assert all(np.array_equal(got[k], want[k]) for k in ("n", "total_candidates", "status"))
+    assert all(np.array_equal(got[k][i, :n], want[k][i, :n]) for k in ("doc_key", "score", "tie") for i, n in enumerate(want["n"]))     # slots after n are undefined
     if multi:
         flt = ib.Filter.Parse("year >= 2000 AND rating > 7.0")
         assert not compare_search(eng, orc, qs[:80], flt=flt, facets=True)
