@@ -182,8 +182,7 @@ struct S1Workspace {
     int32_t* cand;         // sorted candidate ids
     int32_t* buf_a; int32_t* buf_b;   // AND-tier ping-pong arrays
     unsigned long long* surv_g;       // [CHUNK] flush survivors of one chunk when they exceed the shared staging buffer
-    int32_t* rank;         // [n_words ..): padded tf slots before container c (scratch of the tf lookups)
-    unsigned long long* probe;   // per bitset word: (bits, candidates before the word) -- S1Probe, valid between the compaction and the tf lookups; bits all zero between queries
+    int32_t* lrange;       // [MAX_TERMS][n_cont + 1] per streamed list of the tf lookups: index of its first posting in container c
     int32_t* cstart;       // [n_cont + 1] candidates before container c
     int32_t* cfirst;       // [n_cont + 1] chunks before container c
     int32_t* ctab;         // [n_cont] packed S1Cont records (16 bytes each) for the tf lookups

@@ -21,9 +21,20 @@ struct S1Rec {
     int32_t state;                                                            // 0 nothing to score, 1 light / 4 mid (score_warp), 3 heavy (score_cta), 2 deferred (pool full), -1 overflow
     int32_t K, path, pad;
 };
-struct S1Queues { int32_t* light; int32_t* mid; int32_t* heavy; };
-struct alignas(8) S1Probe { unsigned bits; int32_t rank; };                     // one candidate-bitset word and the candidates before it: a posting's probe is ONE 8-byte load
-struct alignas(16) S1Cont { int32_t cstart, cnt, cpad, cfirst; };                // per container: candidates before it, its candidates, padded tf slots before it, chunks before it                           // query ids appended by stage1_lookup (counters in BatchCounters)
+struct S1Queues { int32_t* light; int32_t* mid; int32_t* heavy; };            // query ids appended by stage1_lookup (counters in BatchCounters)
+struct alignas(16) S1Cont { int32_t cstart, cnt, cpad, cfirst; };                // per container: candidates before it, its candidates, padded tf slots before it, chunks before it
+
+// Shared memory of the selection / tf-lookup kernel: the selection's state plus the on-chip slice of the candidate bitset that the
+// streamed tf lookups probe, one 65 536-doc container at a time. (A struct of its own: S1Shared, the scorer's and the LD1
+// expansion's at two CTAs per SM, extends S1SelShared and has no room for the slice.)
+constexpr int CONT_WORDS = 65536 / 32;
+struct S1LookShared : S1SelShared {
+    unsigned cbits[CONT_WORDS];                // the container's bitset words
+    uint16_t crank[CONT_WORDS];                // the container's candidates before each word
+    const int32_t* sdoc[MAX_TERMS]; const uint8_t* stf[MAX_TERMS];   // streamed list j: its postings (and tfs) in the container, from the first one on
+    int slen[MAX_TERMS]; int spre[MAX_TERMS + 1];                      // ... smis + their count, and where they start in the container's flattened range
+    uint8_t smis[MAX_TERMS], slist[MAX_TERMS], srow[MAX_TERMS];        // ... 16-byte misalignment of the first (in postings), its slot in `terms`, its row of the tf matrix
+};
 
 IFX_FN int pad16(int x) { return (x + 15) & ~15; }
 constexpr int DEL_BIT = (int)0x80000000;
@@ -37,12 +48,14 @@ constexpr int W_K = 512;             // heap capacity kept in shared memory per 
 
 // ---------------------------------------------------------------------------------------------------------------
 // stage1_lookup: called right after stage1_select by the same CTA. Candidates are the bits of ws.bits.
-//   1. count + expand the bitset into the pool (ascending ids), building the rank directory (doc -> candidate index in O(1))
+//   1. count + expand the bitset into the pool (ascending ids), candidates before every container
 //   2. document lengths, deleted flags, chunk table
 //   3. tf of every (term, candidate): either every posting list streamed once against the candidate bitset (coalesced; the byte
-//      volume SURVEY 8d calls algorithmic), or -- few candidates relative to the lists -- one forward-index read per candidate
+//      volume SURVEY 8d calls algorithmic), or -- few candidates relative to the lists -- one forward-index read per candidate.
+//      The lists are streamed container by container: the container's 8 KB of bitset and its per-word candidate ranks sit in shared
+//      memory, so a posting's probe never leaves the SM
 //   4. bitset cleared again
-IFX_FN void stage1_lookup(const Ctx& c, const DevIndex& ix, const QueryPlan& p, int path, int q, S1Workspace& ws, S1SelShared& sh, S1Rec* recs,
+IFX_FN void stage1_lookup(const Ctx& c, const DevIndex& ix, const QueryPlan& p, int path, int q, S1Workspace& ws, S1LookShared& sh, S1Rec* recs,
                           unsigned char* spool, unsigned long long spool_cap, S1Queues queues, BatchCounters* bc, Stage1Out out, int fwd_avg_bytes, int force_mode) {
     S1Rec& rec = recs[q]; const int NT = c.nthreads(), NW = c.nwarps(); constexpr int WS = Ctx::WS;
 #if !defined(IFX_EMU) && defined(IFX_S1_TIMERS)
@@ -63,8 +76,7 @@ IFX_FN void stage1_lookup(const Ctx& c, const DevIndex& ix, const QueryPlan& p, 
     }
     int n_cand; int ex0 = block_excl_scan(c, mycnt, sh.scan, n_cand); const int wbase = c.shfl(ex0, 0);
     auto clear_bits = [&]() {
-        S1Probe* pr = reinterpret_cast<S1Probe*>(ws.probe);
-        for (int64_t w = c.tid(); w < nwords; w += NT) if (sh.dirty[w >> 11]) { ws.bits[w] = 0u; pr[w].bits = 0u; }
+        for (int64_t w = c.tid(); w < nwords; w += NT) if (sh.dirty[w >> 11]) ws.bits[w] = 0u;
         c.sync();
         for (int k = c.tid(); k < ncont; k += NT) sh.dirty[k] = 0;
         c.sync();
@@ -80,7 +92,7 @@ IFX_FN void stage1_lookup(const Ctx& c, const DevIndex& ix, const QueryPlan& p, 
     const long long a1 = pool_alloc(8ULL * (unsigned long long)n_cand + 64);
     if (a1 < 0) { give_up(a1); return; }
     int32_t* cand = reinterpret_cast<int32_t*>(spool + a1); float* dlp = reinterpret_cast<float*>(spool + a1 + (((long long)n_cand * 4 + 31) & ~31LL));
-    // ---- 1b. expand + rank directory + candidates before every container
+    // ---- 1b. expand + candidates before every container
     {   int run = wbase;
         for (int64_t gb = w0; gb < w1; gb += 4 * WS) {          // four groups per trip: their words are loaded together, then scanned one after the other
             unsigned vv[4];
@@ -91,7 +103,7 @@ IFX_FN void stage1_lookup(const Ctx& c, const DevIndex& ix, const QueryPlan& p, 
                 const int64_t w = g0 + c.lane(); unsigned v = vv[u]; const int pc = popc(v); int incl = pc;
                 for (int d = 1; d < WS; d <<= 1) { int o = c.shfl(incl, c.lane() >= d ? c.lane() - d : 0); if (c.lane() >= d) incl += o; }
                 int o = run + incl - pc;
-                if (w < w1) { S1Probe pv; pv.bits = v; pv.rank = o; reinterpret_cast<S1Probe*>(ws.probe)[w] = pv; if ((w & 2047) == 0) ws.cstart[w >> 11] = o; }
+                if (w < w1 && (w & 2047) == 0) ws.cstart[w >> 11] = o;
                 while (v) { int b = ffs32(v) - 1; v &= v - 1; cand[o++] = (int32_t)((w << 5) | b); }
                 run += c.shfl(incl, WS - 1);
             }
@@ -99,7 +111,7 @@ IFX_FN void stage1_lookup(const Ctx& c, const DevIndex& ix, const QueryPlan& p, 
         if (c.tid() == 0) ws.cstart[ncont] = n_cand;
     }
     c.sync();
-    IFX_LTICK(0);   // count + expand + rank directory
+    IFX_LTICK(0);   // count + expand
     // ---- 2. lengths, deleted flags (folded into the id), chunk table
     const bool any_deleted = ix.n_live != ix.n_docs;
     for (int i0 = c.tid(); i0 < n_cand; i0 += 8 * NT) {
@@ -118,13 +130,13 @@ IFX_FN void stage1_lookup(const Ctx& c, const DevIndex& ix, const QueryPlan& p, 
         const int cc = c0 + c.tid(); const int cntc = cc < ncont ? ws.cstart[cc + 1] - ws.cstart[cc] : 0;
         const int nch = (cntc + CHUNK - 1) / CHUNK; const int slots = (cntc / CHUNK) * CHUNK + pad16(cntc % CHUNK);
         int t1, t2; const int e1 = block_excl_scan(c, nch, sh.scan, t1); const int e2 = block_excl_scan(c, slots, sh.scan, t2);
-        if (cc < ncont) { ws.cfirst[cc] = n_chunks + e1; ws.rank[nwords + cc] = n_slots + e2;      // padded slots before container cc: kept behind the rank directory
+        if (cc < ncont) { ws.cfirst[cc] = n_chunks + e1;
                           S1Cont ct; ct.cstart = ws.cstart[cc]; ct.cnt = cntc; ct.cpad = n_slots + e2; ct.cfirst = n_chunks + e1; reinterpret_cast<S1Cont*>(ws.ctab)[cc] = ct; }
         if (cntc > 0) atomic_max(&sh.bcast[1], cntc < CHUNK ? cntc : CHUNK);
         n_chunks += t1; n_slots += t2;
     }
     c.sync();
-    const int max_cnt = sh.bcast[1]; const int32_t* cpad = ws.rank + nwords;
+    const int max_cnt = sh.bcast[1]; const S1Cont* ctab = reinterpret_cast<const S1Cont*>(ws.ctab);
     const unsigned long long tf_bytes = (unsigned long long)(Ta > 0 ? Ta : 1) * (unsigned long long)n_slots;
     const unsigned long long chunk_bytes = ((unsigned long long)n_chunks * sizeof(S1Chunk) + 15ULL) & ~15ULL, term_bytes = (unsigned long long)(Ta > 0 ? Ta : 1) * sizeof(S1TermP);
     const long long a2 = pool_alloc(chunk_bytes + term_bytes + tf_bytes + 64);
@@ -133,7 +145,7 @@ IFX_FN void stage1_lookup(const Ctx& c, const DevIndex& ix, const QueryPlan& p, 
     uint8_t* tfb = spool + a2 + chunk_bytes + term_bytes;
     for (int cc = c.tid(); cc < ncont; cc += NT) {
         const int cntc = ws.cstart[cc + 1] - ws.cstart[cc]; const int nch = (cntc + CHUNK - 1) / CHUNK;
-        for (int s = 0; s < nch; s++) { S1Chunk ch; ch.start = ws.cstart[cc] + s * CHUNK; ch.cnt = cntc - s * CHUNK < CHUNK ? cntc - s * CHUNK : CHUNK; ch.tf_off = (int64_t)Ta * (cpad[cc] + s * CHUNK); chunks[ws.cfirst[cc] + s] = ch; }
+        for (int s = 0; s < nch; s++) { S1Chunk ch; ch.start = ws.cstart[cc] + s * CHUNK; ch.cnt = cntc - s * CHUNK < CHUNK ? cntc - s * CHUNK : CHUNK; ch.tf_off = (int64_t)Ta * (ctab[cc].cpad + s * CHUNK); chunks[ws.cfirst[cc] + s] = ch; }
     }
     for (int t = c.tid(); t < T; t += NT) if (sh.order[t] >= 0) { S1TermP tp; tp.idf = sh.terms[t].idf; tp.max_score = sh.terms[t].max_score; tp.suffix_after = sh.terms[t].suffix_after; tp.pad = 0; tparams[sh.order[t]] = tp; }
     {   // zero the tf matrix (16-byte stores; the block is 16-byte aligned and padded)
@@ -146,47 +158,6 @@ IFX_FN void stage1_lookup(const Ctx& c, const DevIndex& ix, const QueryPlan& p, 
     unsigned long long cost_s = 0; int n_dict = 0;
     for (int t = 0; t < T; t++) if (sh.order[t] >= 0 && sh.terms[t].term_id >= 0) { cost_s += 5ULL * (unsigned long long)sh.terms[t].len; n_dict++; }
     const bool forward = force_mode == 1 ? true : (force_mode == 2 ? false : (n_dict > 0 && 3ULL * (unsigned long long)n_cand * (unsigned long long)fwd_avg_bytes < cost_s));      // random forward-list reads cost ~3x a streamed byte (measured, profiles/r2)
-    const S1Cont* ctab = reinterpret_cast<const S1Cont*>(ws.ctab);
-    const S1Probe* probe = reinterpret_cast<const S1Probe*>(ws.probe);
-    auto put_hit = [&](int d, S1Probe pv, int a, uint8_t tfv) {      // candidate d (bit set in pv.bits) of row a
-        const unsigned bit = 1u << (d & 31); const int idx = pv.rank + popc(pv.bits & (bit - 1)); const S1Cont ct = ctab[d >> 16];
-        const int jc = idx - ct.cstart, sub = jc / CHUNK; const int cnt_k = ct.cnt - sub * CHUNK < CHUNK ? ct.cnt - sub * CHUNK : CHUNK;
-        tfb[(int64_t)Ta * (ct.cpad + sub * CHUNK) + (int64_t)a * pad16(cnt_k) + (jc - sub * CHUNK)] = tfv;
-    };
-    auto stream_term = [&](const TermS& tm, int a) {      // every posting of one list against the candidate bitset
-        const int64_t len = tm.len; int64_t done = 0;
-#ifndef IFX_EMU
-        if (len >= 2048) {
-            // aligned middle of the list: 16 postings per thread in flight (four 16-byte id loads + four 4-byte tf loads), then their
-            // 16 bitset probes, then the hits
-            const int64_t pre = (int64_t)((0 - (reinterpret_cast<uintptr_t>(tm.docs) >> 2)) & 3);
-            for (int64_t i = c.tid(); i < pre; i += NT) { const int d = tm.docs[i]; const S1Probe wv = probe[d >> 5]; if ((wv.bits >> (d & 31)) & 1u) put_hit(d, wv, a, tm.tf ? tm.tf[i] : (uint8_t)1); }
-            const int4* p4 = reinterpret_cast<const int4*>(tm.docs + pre); const unsigned* t4 = tm.tf ? reinterpret_cast<const unsigned*>(tm.tf + pre) : nullptr;
-            const int64_t n4 = (len - pre) >> 2;
-            for (int64_t g0 = c.tid(); g0 < n4; g0 += 4LL * NT) {
-                int4 dv[4]; unsigned tw[4]; S1Probe wv[16];
-#pragma unroll
-                for (int u = 0; u < 4; u++) { const int64_t g = g0 + (int64_t)u * NT; if (g < n4) { dv[u] = p4[g]; tw[u] = t4 ? t4[g] : 0x01010101u; } else { dv[u] = make_int4(-1, -1, -1, -1); tw[u] = 0u; } }
-#pragma unroll
-                for (int u = 0; u < 4; u++) { const int dd[4] = {dv[u].x, dv[u].y, dv[u].z, dv[u].w};
-#pragma unroll
-                    for (int k = 0; k < 4; k++) { if (dd[k] >= 0) wv[4 * u + k] = probe[dd[k] >> 5]; else wv[4 * u + k].bits = 0u; } }
-#pragma unroll
-                for (int u = 0; u < 4; u++) { const int dd[4] = {dv[u].x, dv[u].y, dv[u].z, dv[u].w};
-#pragma unroll
-                    for (int k = 0; k < 4; k++) if (dd[k] >= 0 && ((wv[4 * u + k].bits >> (dd[k] & 31)) & 1u)) put_hit(dd[k], wv[4 * u + k], a, (uint8_t)(tw[u] >> (8 * k))); }
-            }
-            done = pre + (n4 << 2);
-        }
-#endif
-        const int64_t NT4 = 4LL * NT;
-        for (int64_t i0 = done + c.tid(); i0 < len; i0 += NT4) {
-            int dd[4]; uint8_t tv[4]; S1Probe wv[4];
-            for (int u = 0; u < 4; u++) { int64_t i = i0 + (int64_t)u * NT; const bool in = i < len; dd[u] = in ? tm.docs[i] : -1; tv[u] = (in && tm.tf) ? tm.tf[i] : (uint8_t)1; }
-            for (int u = 0; u < 4; u++) { if (dd[u] >= 0) wv[u] = probe[dd[u] >> 5]; else wv[u].bits = 0u; }
-            for (int u = 0; u < 4; u++) if (dd[u] >= 0 && ((wv[u].bits >> (dd[u] & 31)) & 1u)) put_hit(dd[u], wv[u], a, tv[u]);
-        }
-    };
     if (forward) {
         // Batches of FW_G candidates per warp: their forward lists (a few dozen to a few hundred (term, tf) pairs each) are walked as ONE
         // concatenated range, so a lane has several independent loads in flight instead of one dependent chain per candidate. The
@@ -208,12 +179,98 @@ IFX_FN void stage1_lookup(const Ctx& c, const DevIndex& ix, const QueryPlan& p, 
                 }
             }
         }
-        for (int t = 0; t < T; t++) if (sh.order[t] >= 0 && sh.terms[t].term_id < 0) stream_term(sh.terms[t], sh.order[t]);      // LD1 unions have no term id
-    } else {
-        for (int t = 0; t < T; t++) if (sh.order[t] >= 0) stream_term(sh.terms[t], sh.order[t]);
+        c.sync();
+        IFX_LTICK(3);   // forward-index lookups
     }
+    // Streamed lists: every scored list, or in forward mode the LD1 unions (they have no term id, hence no forward entries).
+    if (c.tid() == 0) { int ns = 0; for (int t = 0; t < T; t++) if (sh.order[t] >= 0 && (!forward || sh.terms[t].term_id < 0)) { sh.slist[ns] = (uint8_t)t; sh.srow[ns] = (uint8_t)sh.order[t]; ns++; } sh.bcast[2] = ns; }
     c.sync();
-    IFX_LTICK(3);   // tf lookups
+    const int Ts = sh.bcast[2];
+    if (Ts > 0) {
+        // Where each list enters every container: ws.lrange[j][cc], one thread per (list, container) pair. Long dictionary lists read
+        // their skip table; short ones and the LD1 unions (sorted, no skip table) are searched, once per query rather than once per
+        // container inside the loop below. Only the bounds of containers with candidates are needed.
+        const int NC1 = ncont + 1;
+        for (int i = c.tid(); i < Ts * NC1; i += NT) {
+            const int j = i / NC1, cc = i - j * NC1;
+            if (!((cc < ncont && sh.dirty[cc]) || (cc > 0 && sh.dirty[cc - 1]))) continue;
+            const TermS& tm = sh.terms[sh.slist[j]];
+            ws.lrange[i] = tm.skip ? tm.skip[cc] : (int32_t)lower_bound_i32(tm.docs, 0, tm.len, cc << 16);
+        }
+        c.sync();
+        IFX_LTICK(5);   // per-container list ranges
+        // Container-major lookups: the container's bitset words and their candidate ranks go to shared memory; then the container's
+        // postings of all streamed lists, concatenated into one range, are spread over the whole block. A list's part of the range
+        // starts at the 16-byte boundary before its first posting and is padded to whole groups of four, so that a group lies in one
+        // list and, when all four are its postings, is one 16-byte id load plus one 4-byte tf load; LG groups per thread in flight.
+        // A hit's slot follows from the rank within the container and the container's sub-chunk layout.
+        constexpr int LG = 4;
+        struct alignas(16) Id4 { int32_t v[4]; };
+        for (int cc = 0; cc < ncont; cc++) {
+            if (!sh.dirty[cc]) continue;                  // (uniform) never touched: no candidates
+            const S1Cont ct = ctab[cc];
+            if (ct.cnt == 0) continue;
+            const unsigned* bw = ws.bits + (int64_t)cc * CONT_WORDS;      // (the bitset is allocated to whole containers)
+            for (int w = c.tid(); w < CONT_WORDS; w += NT) sh.cbits[w] = bw[w];
+            for (int j = c.tid(); j < Ts; j += NT) {
+                const TermS& tm = sh.terms[sh.slist[j]]; const int32_t r0 = ws.lrange[j * NC1 + cc], n = ws.lrange[j * NC1 + cc + 1] - r0;
+                const int32_t* dp = tm.docs + r0; const int m = (int)((reinterpret_cast<uintptr_t>(dp) >> 2) & 3);
+                sh.sdoc[j] = dp - m; sh.stf[j] = tm.tf ? tm.tf + r0 - m : nullptr; sh.smis[j] = (uint8_t)m; sh.slen[j] = n > 0 ? m + n : 0;
+            }
+            c.sync();
+            {   // exclusive candidate rank of every word: each thread owns `per` consecutive words
+                const int per = (CONT_WORDS + NT - 1) / NT, w0 = c.tid() * per; int mine = 0, tot;
+                for (int k = 0; k < per && w0 + k < CONT_WORDS; k++) mine += popc(sh.cbits[w0 + k]);
+                int r = block_excl_scan(c, mine, sh.scan, tot);
+                for (int k = 0; k < per && w0 + k < CONT_WORDS; k++) { sh.crank[w0 + k] = (uint16_t)r; r += popc(sh.cbits[w0 + k]); }
+            }
+            {   // start of every list's padded part in the concatenated range
+                const int per = (Ts + NT - 1) / NT, j0 = c.tid() * per; int mine = 0, E;
+                for (int k = 0; k < per && j0 + k < Ts; k++) mine += (sh.slen[j0 + k] + 3) & ~3;
+                int r = block_excl_scan(c, mine, sh.scan, E);
+                for (int k = 0; k < per && j0 + k < Ts; k++) { sh.spre[j0 + k] = r; r += (sh.slen[j0 + k] + 3) & ~3; }
+                if (c.tid() == 0) sh.spre[Ts] = E;
+            }
+            c.sync();
+            const int G = sh.spre[Ts] >> 2; int j = 0;
+            for (int g0 = c.tid(); g0 < G; g0 += LG * NT) {
+                Id4 dv[LG]; unsigned tw[LG]; const int jr = j;      // a group's docs (-1: not a posting of the list) and tfs; the list index at the first group
+#pragma unroll
+                for (int u = 0; u < LG; u++) {
+                    const int g = g0 + u * NT; tw[u] = 0u;
+#pragma unroll
+                    for (int x = 0; x < 4; x++) dv[u].v[x] = -1;
+                    if (g < G) {
+                        while (4 * g >= sh.spre[j + 1]) j++;      // (groups of a thread ascend: the list index only moves forward)
+                        const int k = 4 * g - sh.spre[j], lo = sh.smis[j], hi = sh.slen[j]; const int32_t* dp = sh.sdoc[j] + k; const uint8_t* tp = sh.stf[j];
+                        if (k >= lo && k + 4 <= hi) { dv[u] = *reinterpret_cast<const Id4*>(dp); tw[u] = tp ? *reinterpret_cast<const unsigned*>(tp + k) : 0x01010101u; }
+                        else {
+#pragma unroll
+                            for (int x = 0; x < 4; x++) if (k + x >= lo && k + x < hi) { dv[u].v[x] = dp[x]; tw[u] |= (tp ? (unsigned)tp[k + x] : 1u) << (8 * x); }
+                        }
+                    }
+                }
+                j = jr;      // walked again for the rows: cheaper than holding them across the loads
+#pragma unroll
+                for (int u = 0; u < LG; u++) {
+                    const int g = g0 + u * NT; if (g >= G) break;
+                    while (4 * g >= sh.spre[j + 1]) j++;
+                    const int64_t row = sh.srow[j];
+#pragma unroll
+                    for (int x = 0; x < 4; x++) {
+                        const int d = dv[u].v[x]; if (d < 0) continue;
+                        const int w = (d >> 5) & (CONT_WORDS - 1); const unsigned bits = sh.cbits[w], bit = 1u << (d & 31);
+                        if (bits & bit) {
+                            const int jc = sh.crank[w] + popc(bits & (bit - 1)), sub = jc / CHUNK; const int cnt_k = ct.cnt - sub * CHUNK < CHUNK ? ct.cnt - sub * CHUNK : CHUNK;
+                            tfb[(int64_t)Ta * (ct.cpad + sub * CHUNK) + row * pad16(cnt_k) + (jc - sub * CHUNK)] = (uint8_t)(tw[u] >> (8 * x));
+                        }
+                    }
+                }
+            }
+            c.sync();                                     // the slice is rewritten for the next container
+        }
+        IFX_LTICK(6);   // container-major streamed lookups
+    }
     // ---- 4. bitset back to all-zero; record, queue, roofline accounting (SURVEY 8d)
     clear_bits();
     IFX_LTICK(4);   // bitset cleared

@@ -25,6 +25,6 @@ for i in order[:8]: print("%-36s cand=%7d T=%3d path=%d mode=%d chunks=%4d maxcn
 order = np.argsort(-k2)
 for i in order[:5]: print("K2 top: %-30s cand=%7d T=%3d chunks=%4d maxcnt=%4d light=%d K2=%.2f ms" % (qs[i][:30], nc[i], ta[i], nch[i], mx[i], light[i], k2[i]))
 
-if dbg[:, 11:16].sum() > 0:
+if dbg[:, 11:18].sum() > 0:
     for name, sel in (("forward", mode == 1), ("stream", mode == 2)):
-        if sel.any(): print(name, "lookup phases, mean kcycles [count+expand, lengths, chunk table+zero, tf lookups, clear]:", (dbg[sel, 11:16].mean(0) / 1e3).astype(int), "| selection sticks [sort, tier0/unions, tier1, -]:", (dbg[sel, 20:24].mean(0) / 1e3).astype(int))
+        if sel.any(): print(name, "lookup phases, mean kcycles [count+expand, lengths, chunk table+zero, forward-index lookups, clear, list ranges, streamed lookups]:", (dbg[sel, 11:18].mean(0) / 1e3).astype(int), "| selection sticks [sort, tier0/unions, tier1, -]:", (dbg[sel, 20:24].mean(0) / 1e3).astype(int))
